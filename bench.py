@@ -370,9 +370,9 @@ def dropin_rate(w, device, n=200_000):
                           'wire_bytes_per_row': len(sent[0])}}
 
 
-def measure_prss(w, n, steps, warmup, local, rank, peak, with_e2e=True):
+def measure_prss(w, n, steps, warmup, local, rank, peak, with_e2e=True, dump_dir=None, dump_suffix=''):
     """K4 on PRF bytes resident in HBM (CUDA events), and -- with_e2e -- the host pipeline mpyc_b200_prss_host and the
-    drop-in call at np_cnnmnist's largest per-call size."""
+    drop-in call at np_cnnmnist's largest per-call size.  dump_dir: write the shares of the last timed step there."""
     import itertools
     import numpy as np
     import torch
@@ -416,6 +416,8 @@ def measure_prss(w, n, steps, warmup, local, rank, peak, with_e2e=True):
     t_end = time.perf_counter()
     launches = mpyc_b200.launch_count() - launches0
     ms = ev[0].elapsed_time(ev[-1]) / steps
+    if dump_dir:
+        dump_outputs(dump_dir, {'prss_shares': d_out.unsqueeze(0)}, n, dump_suffix)
     alg = n * (nsub * d * chunk + eb)
     ach = alg / (ms * 1e-3) / 1e9
     out = {'kernel': 'k_prss_tiles', 'n': n, 'subsets': nsub, 'chunk_bytes': chunk, 'ms': ms, 'algorithmic_bytes': alg,
@@ -465,7 +467,7 @@ def run_prss_arm(a, w):
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    r = measure_prss(w, n, a.steps, a.warmup, local, rank, peak)
+    r = measure_prss(w, n, a.steps, a.warmup, local, rank, peak, dump_dir=a.dump_outputs, dump_suffix=rank_suffix(world, rank))
     ms = r['ms']
     if world > 1:
         tt = torch.tensor([ms], device='cuda')
@@ -526,9 +528,33 @@ def _dist_init(local):
     return dist
 
 
-def measure_device(w, n, steps, warmup, seed_rank=0, sustain_s=0.0, keep=False):
+DUMP_SAMPLE = 1 << 16       # elements per output written by --dump-outputs (at most ~34 MB in all, for c5)
+
+
+def dump_outputs(directory, arrays, n, suffix=''):
+    """--dump-outputs: write device outputs as DIR/<name><suffix>.npy.  `arrays` maps names to tensors whose axis 1 is
+    the element axis: int64 limbs (rows, n, L) or GF(2^8) bytes (rows, n).  Limbs become float64 words, exactly: each
+    64-bit limb is split into two 32-bit words, least significant first, so an element is 2L words.  GF(2^8) bytes
+    become float32.  Outputs longer than DUMP_SAMPLE elements are sampled at seeded element indices, the same in every
+    run and every array, and element_index<suffix>.npy records them."""
+    import numpy as np
+    import torch
+    os.makedirs(directory, exist_ok=True)
+    if n > DUMP_SAMPLE:
+        idx = np.unique(np.random.default_rng(20260923).integers(0, n, size=DUMP_SAMPLE))
+    else:
+        idx = np.arange(n)
+    np.save(os.path.join(directory, f'element_index{suffix}.npy'), idx.astype(np.float64))
+    for name, t in arrays.items():
+        x = t.index_select(1, torch.from_numpy(idx).to(t.device)).cpu().numpy()
+        x = x.astype(np.float32) if x.dtype == np.uint8 else x.view(np.uint32).astype(np.float64)
+        np.save(os.path.join(directory, f'{name}{suffix}.npy'), x[0] if x.shape[0] == 1 else x)
+
+
+def measure_device(w, n, steps, warmup, seed_rank=0, sustain_s=0.0, keep=False, dump_dir=None, dump_suffix=''):
     """K steps of the hot path on device-resident inputs, timed with CUDA events on the launching stream.
-    Returns a dict with per-kernel milliseconds, launches and (keep=True) the buffers for later checks."""
+    Returns a dict with per-kernel milliseconds, launches and (keep=True) the buffers for later checks.
+    dump_dir: write the outputs of the last timed step there (dump_outputs)."""
     import torch
     import mpyc_b200
     from mpyc_b200 import _cabi, device as dev
@@ -586,6 +612,9 @@ def measure_device(w, n, steps, warmup, seed_rank=0, sustain_s=0.0, keep=False):
     common = dict(ctx=ctx, is_mul=is_mul, eb=ctx.elem_bytes, L=max(ctx.nlimbs, 1))
     res = timed(steps)
     res.update(common)
+    if dump_dir:
+        outputs = {'product': OUT.t.unsqueeze(0)} if is_mul else {'shares': SH.t, 'recombined': REC.t}
+        dump_outputs(dump_dir, outputs, n, dump_suffix)
     if sustain_s > 0:
         per = max(res['total_ms'] / steps, 1e-3)
         res['sustained'] = timed(max(steps, int(sustain_s * 1e3 / per) + 1))
@@ -803,6 +832,11 @@ def pcie_probe(nbytes=1 << 29, reps=3):
             'bytes_per_copy': nbytes}
 
 
+def rank_suffix(world, rank):
+    """With N > 1 every rank dumps its own shard of the element axis."""
+    return f'_rank{rank}' if world > 1 else ''
+
+
 def run_gpu_arm(a, w):
     local = int(os.environ.get('LOCAL_RANK', '0'))
     numa = bind_to_gpu_numa(local)       # before CUDA initialisation and any pinned allocation
@@ -838,7 +872,8 @@ def run_gpu_arm(a, w):
     if world > 1:
         dist.barrier()
     torch.cuda.synchronize()
-    res = measure_device(w, n, a.steps, a.warmup, seed_rank=rank, sustain_s=a.sustain, keep=True)
+    res = measure_device(w, n, a.steps, a.warmup, seed_rank=rank, sustain_s=a.sustain, keep=True,
+                         dump_dir=a.dump_outputs, dump_suffix=rank_suffix(world, rank))
     if world > 1:
         dist.barrier()
     is_mul, eb, L, ctx = res['is_mul'], res['eb'], res['L'], res['ctx']
@@ -1073,7 +1108,11 @@ def main():
     ap.add_argument('--no-selftest', action='store_true', help='skip the multi-GPU pre-flight and the gather timing (N > 1)')
     ap.add_argument('--sustain', type=float, default=2.0, help='seconds of the sustained pass after the K timed steps (0 = off)')
     ap.add_argument('--config', dest='workload_alias', default=None, help='alias of --workload')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the outputs of the last timed step to DIR/<name>.npy (GPU arm; see dump_outputs)')
     a = ap.parse_args()
+    if a.dump_outputs and a.impl != 'ours':
+        ap.error('--dump-outputs applies to the GPU arm (--impl ours)')
     if a.workload_alias:
         a.workload = a.workload_alias
     a.warmup = max(a.warmup, 3) if a.impl == 'ours' else a.warmup

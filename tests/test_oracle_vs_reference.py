@@ -1,133 +1,118 @@
-"""Live cross-check of the oracle against the UNMODIFIED reference (only where /root/reference exists, i.e. the build
-container): beyond the committed golden fixtures, randomised (p, m, t, n) instances of every function on the path --
-split (np and list order), recombination vectors and recombination, f_S(i), PRF, PRSS shares and zero-shares, and the
-field-array operators -- with secrets.randbelow replaced by a fixed stream for the duration of each reference call."""
+"""Cross-check of the oracle against the UNMODIFIED reference on randomised (p, m, t, n) instances of every function on
+the path, beyond the edge cases of the other golden fixtures -- split (np and list order), recombination vectors and
+recombination, f_S(i), PRF, PRSS shares and zero-shares, the field-array operators and the protocols' local algebra.
+The instances come from the seeded generators below; what the reference returned on them (secrets.randbelow replaced
+by the instance's fixed stream for the duration of each call) is stored in tests/golden/random_instances.json, written
+by tests/golden/make_golden_random.py."""
 import itertools
-import os
 import random
-import sys
 
 import pytest
 
-REF = os.environ.get('MPYC_REFERENCE', '/root/reference')
-if not os.path.isdir(os.path.join(REF, 'mpyc')):
-    pytest.skip('reference checkout not present', allow_module_level=True)
-
-from oracle import shamir_oracle as orc   # noqa: E402
-
-
-@pytest.fixture(scope='module')
-def ref():
-    sys.dont_write_bytecode = True
-    sys.path.insert(0, REF)
-    argv, sys.argv = sys.argv, [sys.argv[0], '--no-log']
-    try:
-        from mpyc import thresha, finfields, gfpx
-    finally:
-        sys.argv = argv
-    yield thresha, finfields, gfpx
-    sys.path.remove(REF)
-
-
-class injected:
-    def __init__(self, thresha, stream):
-        self.thresha, self.it = thresha, iter(stream)
-
-    def __enter__(self):
-        self.orig = self.thresha.secrets.randbelow
-        self.thresha.secrets.randbelow = lambda order: next(self.it)
-
-    def __exit__(self, *exc):
-        self.thresha.secrets.randbelow = self.orig
-
+from golden_util import load, unhex
+from oracle import shamir_oracle as orc
 
 PRIMES = [2**61 - 1, 2**64 - 189, 2**69 - 93, 2**128 - 173, 2**256 - 189, 9409569905028393239, 101, 2**89 - 1]
 
 
-@pytest.mark.parametrize('p', PRIMES, ids=lambda p: f'p{p.bit_length()}')
-def test_split_recombine_prss_random_instances(ref, p):
-    import numpy as np
-    thresha, finfields, gfpx = ref
-    F, Fo = finfields.GF(p), orc.field_of(p)
+def split_instances(p):
     rnd = random.Random(p % 10007)
     for m, t in ((1, 0), (3, 1), (4, 1), (5, 2), (7, 3), (6, 5)):
         n = rnd.randrange(1, 9)
         s = [rnd.randrange(p) for _ in range(n)]
         stream = [rnd.randrange(p) for _ in range(t * n)]
-        with injected(thresha, stream):
-            sh_np = thresha.np_random_split(F, F.array(np.array(s, dtype=object)), t, m)
-        C_np = orc.np_stream_to_C(stream, t, n)
-        assert sh_np.tolist() == orc.split_np_order(Fo, s, C_np, m)
-        with injected(thresha, stream):
-            sh_li = thresha.random_split(F, [F(x) for x in s], t, m)
-        assert sh_li == orc.split_list_order(Fo, s, orc.list_stream_to_c(stream, t, n), m)
         xs = sorted(rnd.sample(range(1, m + 1), min(m, t + 1)))
-        for x_r in (0, m + 1):
-            assert [int(v) % p for v in thresha._recombination_vector(F, tuple(xs), x_r)] == orc.recombination_vector(Fo, xs, x_r)
-        y = thresha.np_recombine(F, [(x, sh_np[x - 1]) for x in xs])
-        assert y.value.tolist() == orc.recombine(Fo, xs, [sh_np[x - 1].tolist() for x in xs]) == s
-        # PRSS for one party
         i = rnd.randrange(m)
         subsets = [S for S in itertools.combinations(range(m), m - t) if i in S]
         keys = {S: bytes(rnd.randrange(256) for _ in range(16)) for S in subsets}
-        prfs = {S: thresha.PRF(k, p) for S, k in keys.items()}
         uci = bytes(rnd.randrange(256) for _ in range(5))
-        for S in subsets:
-            assert int(thresha._f_S_i(F, m, i, S)) % p == orc.f_S_i(Fo, m, i, S) % p
-        got = thresha.np_pseudorandom_share(F, m, i, prfs, uci, n).value.tolist()
-        assert got == orc.prss_share(Fo, m, i, {S: orc.prf_values(k, p, uci, n) for S, k in keys.items()}, n)
-        if t:
-            d = t
-            prl = {S: orc.prf_values(k, p, uci, n * d) for S, k in keys.items()}
-            assert thresha.np_pseudorandom_share_0(F, m, i, prfs, uci, n).value.tolist() == orc.prss_share_zero_np_order(Fo, m, i, prl, n)
-            assert [a.value for a in thresha.pseudorandom_share_zero(F, m, i, prfs, uci, n)] == orc.prss_share_zero_list_order(Fo, m, i, prl, n)
+        yield dict(m=m, t=t, n=n, s=s, stream=stream, xs=xs, i=i, keys=keys, uci=uci)
 
 
-@pytest.mark.parametrize('p', PRIMES, ids=lambda p: f'p{p.bit_length()}')
-def test_field_array_operators_random_instances(ref, p):
-    import numpy as np
-    thresha, finfields, gfpx = ref
-    F = finfields.GF(p)
+def operator_instance(p):
     rnd = random.Random(p % 7919)
     a = [rnd.randrange(p) for _ in range(12)]
     b = [rnd.randrange(1, p) for _ in range(12)]
-    A, B = F.array(np.array(a, dtype=object)), F.array(np.array(b, dtype=object))
-    assert (A + B).value.tolist() == orc.ff_add(p, a, b)
-    assert (A - B).value.tolist() == orc.ff_sub(p, a, b)
-    assert (A * B).value.tolist() == orc.ff_mul(p, a, b)
-    assert (-A).value.tolist() == orc.ff_neg(p, a)
-    assert B.reciprocal().value.tolist() == orc.ff_inv(p, b)
-    assert (A / B).value.tolist() == orc.ff_div(p, a, b)
-    assert (A << 5).value.tolist() == orc.ff_lshift(p, a, 5)
-    assert (A >> 5).value.tolist() == orc.ff_rshift(p, a, 5)
-    assert (A ** 7).value.tolist() == orc.ff_pow(p, a, 7)
+    return a, b
 
 
-@pytest.mark.parametrize('p', PRIMES, ids=lambda p: f'p{p.bit_length()}')
-def test_local_algebra_random_instances(ref, p):
-    """oracle.local_* against the expressions of np_random_bits / np_trunc / np_sgn / np_to_bits (mpyc/runtime.py:860,
-    870, 3646-3660, 4252-4271, 4415) evaluated on the reference's field arrays, random sizes and bit counts."""
-    import numpy as np
-    thresha, finfields, gfpx = ref
-    Zp = finfields.GF(p)
+def local_instances(p):
     rnd = random.Random(p % 9973)
-    arr = lambda v: Zp.array(np.array(v, dtype=object))   # noqa: E731
     for _ in range(6):
         n, f = rnd.randrange(1, 7), rnd.randrange(1, 75)
         a, b, c = ([rnd.randrange(p) for _ in range(n)] for _ in range(3))
-        A, B, C = arr(a), arr(b), arr(c)
-        assert Zp.array(A.value**2 + C.value).value.tolist() == orc.local_fma(p, a, a, c)
-        assert Zp.array(A.value * B.value + C.value).value.tolist() == orc.local_fma(p, a, b, c)
         s, t = rnd.randrange(p), rnd.randrange(p)
-        assert Zp.array(A.value * s + t).value.tolist() == orc.local_axpb(p, a, s, t)
         nb = rnd.randrange(0, p.bit_length() + 3)
-        assert (C.value & ((1 << nb) - 1)).tolist() == orc.local_low_bits(c, nb)
-        assert (A.value != 0).tolist() == orc.local_nonzero(a)
         bits = [rnd.randrange(p) for _ in range(n * f)]
-        R = arr(bits)
-        asc = Zp.array(np.sum(R.value.reshape((n, f)) << np.arange(f), axis=1)).value.tolist()
-        desc = Zp.array(np.sum(R.value.reshape((n, f)) << np.arange(f - 1, -1, -1), axis=1)).value.tolist()
-        assert asc == orc.local_bits_compose(p, bits, n, f) and desc == orc.local_bits_compose(p, bits, n, f, descending=True)
         l = rnd.randrange(1, p.bit_length() + 1)
-        assert (np.right_shift.outer(C.value, np.arange(l - 1, -1, -1)).T & 1).tolist() == orc.local_bits_decompose(c, l, descending=True)
-        assert (np.right_shift.outer(C.value, np.arange(l)).T & 1).tolist() == orc.local_bits_decompose(c, l)
+        yield dict(n=n, f=f, a=a, b=b, c=c, s=s, t=t, nb=nb, bits=bits, l=l)
+
+
+def bit_rows(rows):
+    """A 0/1 matrix as stored in the fixture: one string of '0' and '1' per row."""
+    return [''.join(map(str, r)) for r in rows]
+
+
+@pytest.fixture(scope='module')
+def golden():
+    return load('random_instances.json')['primes']
+
+
+@pytest.mark.parametrize('p', PRIMES, ids=lambda p: f'p{p.bit_length()}')
+def test_split_recombine_prss_random_instances(golden, p):
+    Fo = orc.field_of(p)
+    cases = golden[hex(p)]['split']
+    instances = list(split_instances(p))
+    assert len(cases) == len(instances)
+    for inst, g in zip(instances, cases):
+        m, t, n, s, stream, xs, i = (inst[k] for k in ('m', 't', 'n', 's', 'stream', 'xs', 'i'))
+        sh_np = unhex(g['shares_np'])
+        assert sh_np == orc.split_np_order(Fo, s, orc.np_stream_to_C(stream, t, n), m)
+        assert unhex(g['shares_list']) == orc.split_list_order(Fo, s, orc.list_stream_to_c(stream, t, n), m)
+        for x_r, want in zip((0, m + 1), g['lambda']):
+            assert unhex(want) == orc.recombination_vector(Fo, xs, x_r)
+        assert unhex(g['recombined']) == orc.recombine(Fo, xs, [sh_np[x - 1] for x in xs]) == s
+        # PRSS for one party
+        keys, uci = inst['keys'], inst['uci']
+        for S in keys:
+            assert unhex(g['f_S_i'][','.join(map(str, S))]) == orc.f_S_i(Fo, m, i, S) % p
+        assert unhex(g['prss']) == orc.prss_share(Fo, m, i, {S: orc.prf_values(k, p, uci, n) for S, k in keys.items()}, n)
+        if t:
+            prl = {S: orc.prf_values(k, p, uci, n * t) for S, k in keys.items()}
+            assert unhex(g['zero_np']) == orc.prss_share_zero_np_order(Fo, m, i, prl, n)
+            assert unhex(g['zero_list']) == orc.prss_share_zero_list_order(Fo, m, i, prl, n)
+
+
+@pytest.mark.parametrize('p', PRIMES, ids=lambda p: f'p{p.bit_length()}')
+def test_field_array_operators_random_instances(golden, p):
+    a, b = operator_instance(p)
+    g = {k: unhex(v) for k, v in golden[hex(p)]['operators'].items()}
+    assert g['add'] == orc.ff_add(p, a, b)
+    assert g['sub'] == orc.ff_sub(p, a, b)
+    assert g['mul'] == orc.ff_mul(p, a, b)
+    assert g['neg'] == orc.ff_neg(p, a)
+    assert g['reciprocal'] == orc.ff_inv(p, b)
+    assert g['div'] == orc.ff_div(p, a, b)
+    assert g['lshift5'] == orc.ff_lshift(p, a, 5)
+    assert g['rshift5'] == orc.ff_rshift(p, a, 5)
+    assert g['pow7'] == orc.ff_pow(p, a, 7)
+
+
+@pytest.mark.parametrize('p', PRIMES, ids=lambda p: f'p{p.bit_length()}')
+def test_local_algebra_random_instances(golden, p):
+    """oracle.local_* against the expressions of np_random_bits / np_trunc / np_sgn / np_to_bits (mpyc/runtime.py:860,
+    870, 3646-3660, 4252-4271, 4415) evaluated on the reference's field arrays, random sizes and bit counts."""
+    cases = golden[hex(p)]['local']
+    instances = list(local_instances(p))
+    assert len(cases) == len(instances)
+    for inst, g in zip(instances, cases):
+        n, f, a, b, c, bits, l = (inst[k] for k in ('n', 'f', 'a', 'b', 'c', 'bits', 'l'))
+        assert unhex(g['square_add']) == orc.local_fma(p, a, a, c)
+        assert unhex(g['fma']) == orc.local_fma(p, a, b, c)
+        assert unhex(g['axpb']) == orc.local_axpb(p, a, inst['s'], inst['t'])
+        assert unhex(g['low_bits']) == orc.local_low_bits(c, inst['nb'])
+        assert g['nonzero'] == orc.local_nonzero(a)
+        assert unhex(g['compose_asc']) == orc.local_bits_compose(p, bits, n, f)
+        assert unhex(g['compose_desc']) == orc.local_bits_compose(p, bits, n, f, descending=True)
+        assert g['decompose_desc'] == bit_rows(orc.local_bits_decompose(c, l, descending=True))
+        assert g['decompose_asc'] == bit_rows(orc.local_bits_decompose(c, l))
